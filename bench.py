@@ -1,13 +1,19 @@
 #!/usr/bin/env python
-"""Benchmark of the OpenIBL hot path on B200 (contract: see the task prompt / DESIGN.md).
+"""Benchmark of the OpenIBL hot path on B200 (see DESIGN.md).
 
     python bench.py [--gpus N --steps K --warmup W]          # B200 engine (libiblb200.so)
     python bench.py --impl reference [...]                   # reference CPU arithmetic (oracle port)
+    python bench.py [...] --dump-outputs DIR                 # also save what the timed calls returned
 
 Primary metric (BASELINE.json): images/sec of VGG16+NetVLAD+PCA descriptor extraction at batch 32,
 3x480x640 synthetic images (configs[1]).  The same JSON line carries the retrieval metric
 (query x database pairs/sec, 6.8k x 10k x 4096-d, configs[2]) under "retrieval".
-A step = one batch of 32 images through the whole extraction path.
+A step = one batch of 32 images through the whole extraction path; --steps K times exactly K of them.
+
+--dump-outputs DIR writes rank 0's results of the last timed step as DIR/<name>.npy (1.3 MB in all):
+descriptors.npy (float32 [32, 4096], Engine.extract with PCA) and retrieval_topk_dist.npy /
+retrieval_topk_idx.npy (float32 / float64 [6800, 10], sharded_topk).  Inputs and weights are seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -257,8 +263,14 @@ def main():
     ap.add_argument("--strong-db", type=int, default=250000)
     ap.add_argument("--strong-budget-s", type=float, default=240.0,
                     help="skip the strong-scaling leg if its projected extraction time exceeds this")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed extraction and retrieval steps to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to the B200 engine, not to --impl reference")
         return run_reference(args)
 
     import torch.distributed as dist
@@ -304,10 +316,12 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(args.steps):
-        eng.extract(xs[i % 2], pca=True)
+        desc, _ = eng.extract(xs[i % 2], pca=True)
     e1.record()
     torch.cuda.synchronize()
     launches = eng.launch_count - l0
+    dumped = {"descriptors": desc.cpu()}
+    del desc
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
     barrier()
     clocks = sampler.stop() if rank == 0 else None
@@ -441,9 +455,11 @@ def main():
     r0.record()
     rsteps = 3
     for _ in range(rsteps):
-        sharded_topk(qd, dbd, TOPK, idx_base=rank * NDB, n_valid=NDB)
+        top_d, top_i = sharded_topk(qd, dbd, TOPK, idx_base=rank * NDB, n_valid=NDB)
     r1.record()
     torch.cuda.synchronize()
+    dumped["retrieval_topk_dist"], dumped["retrieval_topk_idx"] = top_d.cpu(), top_i.cpu().double()
+    del top_d, top_i
     r_ms = torch.tensor([r0.elapsed_time(r1) / rsteps], device=dev)
     if world > 1:
         dist.all_reduce(r_ms, op=dist.ReduceOp.MAX)
@@ -522,6 +538,11 @@ def main():
                                     "thread_sweep_images_per_s": {str(k): round(r, 3) for k, r in rates.items()},
                                     "sample": f"8 of the 32 images of one step after a full warm-up pass, oracle "
                                               f"EmbedNetPCA forward, {dt:.1f} s, best thread count of the sweep"}
+        if args.dump_outputs:
+            import numpy as np
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, t in dumped.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), t.numpy())
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
