@@ -195,7 +195,11 @@ int ibl_l2dist_dense(ibl_engine* e, const float* q, int m, const float* db, int 
  * np.argsort (evaluators.py:127-129,143) for the ranks evaluate_all reads (:151-159).
  * out_dist [m,k] ascending, out_idx [m,k] = idx_base + row in db; ties: lowest index first.
  * n_valid <= n rows of db are real (the rest is DistributedSliceSampler padding,
- * sampler.py:208-219, and is ignored).  k <= 128. */
+ * sampler.py:208-219, and is ignored).  k <= 128.  Tensor cores screen, exact fp32 decides: only the
+ * candidates a screening pass keeps are re-scored exactly, and a guard with a bound that holds for any input
+ * (representation errors, accumulator truncation, fp32 rounding) sends every query whose ranking the screening could
+ * have changed to an exact brute force on the device, without host synchronisation.  With k >= 121 the bf16x3 path
+ * keeps fewer than 8 spare candidates, and most queries take that brute force. */
 int ibl_l2dist_topk(ibl_engine* e, const float* q, int m, const float* db, int n, int n_valid,
                     int d, int k, int64_t idx_base, float* out_dist, int64_t* out_idx,
                     void* stream);
@@ -221,8 +225,8 @@ int ibl_gemm_nt(ibl_engine* e, const float* A, int m, const float* B, int n, int
                 void* stream);
 
 /* ---- self-tests (GPU) ------------------------------------------------------ */
-/* Queries that the guard of the single-pass distance path re-ranked by exact brute force in the last
- * ibl_l2dist_topk call (-1: that path was not taken).  Synchronises. */
+/* Queries that the screening guard re-ranked by exact brute force in the last ibl_l2dist_topk call, whichever
+ * tensor-core path it took (-1: the call took the CUDA-core path).  Synchronises. */
 int ibl_debug_dist_flagged(ibl_engine* e, int* count, void* stream);
 /* Runs the tcgen05/TMA building blocks against CUDA-core results on the device;
  * returns IBL_OK when all agree. max_rel_err (may be NULL) receives the worst error. */

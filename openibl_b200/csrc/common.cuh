@@ -51,6 +51,26 @@ struct DeviceOnce {
   void mark() { const int d = cur(); mask[d >> 6].fetch_or(1ull << (d & 63), std::memory_order_release); }
 };
 
+// Screening guard of the distance/top-k paths: an upper bound on |e(q,d) - s(q,d)| for ANY database row d, where
+// e = fmaf(-2, q.d, |q|^2 + |d|^2) with an fp32 dot product (lane-strided FMAs, d/32 per lane, then a 5-level tree)
+// and s = |q|^2 + |d|^2 - 2 q'.d' with q', d' the tensor-core representations, accumulated in TMEM.
+//   representation:  q.d - q'.d' = dq.d' + q'.dd + dq.dd (+ the product the bf16x3 split drops, ql.dl)
+//                    |.| <= |dq||d| + |q||dd| + |dq||dd| (+ |ql||dl|), all |x - x'| computed exactly per row;
+//   accumulation:    the fp32 TMEM accumulator truncates once per MMA; every partial sum is <= |q'||d'|;
+//   fp32 rounding:   of both the dot product and the two distance expressions.
+// an = |q|^2, qe = |q - q'|, dmax_sq / dmax_err = max over the database rows of |d|^2 and |d - d'|,
+// n_mma = MMAs accumulated per dot product, lolo = bound of |ql||dl| / (|q||d|) (0 for the fp16 plane).
+// SCREEN_MMA_REL: the per-MMA truncation measured for kind::bf16 is 1.32e-8 of the accumulator
+// (profiles/r01_diag_tc_accumulator_bias.txt, mean over 108..864 MMAs); 2^-22 = 2 fp32 ulps is 18x that.
+#define SCREEN_MMA_REL 2.3841858e-7f
+__host__ __device__ __forceinline__ float screen_guard_bound(float an, float qe, float dmax_sq, float dmax_err, int d,
+                                                             int n_mma, float lolo) {
+  const float nq = sqrtf(an) * 1.001f, nd = sqrtf(dmax_sq) * 1.001f;   // 1.001: fp32 sums and sqrt of the norms
+  const float rep = qe * nd + nq * dmax_err + qe * dmax_err;
+  const float rel = lolo + (float)n_mma * SCREEN_MMA_REL * 1.01f + (float)(d / 32 + 8) * 5.9604645e-8f;
+  return 1.001f * (2.f * (rep + rel * nq * nd) + 4.7683716e-7f * (an + dmax_sq));   // 2^-21 (|q|^2 + |d|^2)
+}
+
 // SM count of the calling thread's current device
 static inline int device_sm_count() {
   int dev = 0, sms = 0;
@@ -157,14 +177,28 @@ int launch_dist_top16_2sm(const __nv_bfloat16* q_hi, const __nv_bfloat16* q_lo, 
 size_t dist1_workspace_bytes(int m, int n, int d, size_t* off /*[9]*/);
 int launch_dist_topk_1pass(const float* q, int m, const float* db, int n, int n_valid, int d, int k, long long idx_base,
                            void* ws, float* out_dist, long long* out_idx, uint64_t* launches, cudaStream_t s);
-int dist1_last_flag_count(void* ws, int m, int n, int d, int* out, cudaStream_t s);
+int* dist1_flag_count(void* ws, int m, int n, int d);
+int launch_dist_colmax(const float* sq, const float* err, int stride, int n, float* out2, cudaStream_t s);
+size_t dist_exact_scratch_bytes(int m, int n_valid, int k);
+int launch_dist_exact_fallback(const float* q, const float* qn, int qn_stride, int m, const float* db, const float* dbn,
+                               int dbn_stride, int n_valid, int d, int k, long long idx_base, const int* flag_count,
+                               const int* flag_list, unsigned long long* scratch, float* out_dist, long long* out_idx,
+                               cudaStream_t s);
 int pca_tc_splits(int P, int D);
 int launch_pca_partial_tc(const __nv_bfloat16* w_hi, const __nv_bfloat16* w_lo, int P,
                           const __nv_bfloat16* v_hi, const __nv_bfloat16* v_lo, int N, int D,
                           float* partial, int* splits_out, cudaStream_t s);
+// guard inputs of launch_rescore_sort: the bf16x3 representation errors and the screened candidate distances
+struct RescoreGuard {
+  const float* cand_sd;   // [m][kc] screened distances of the candidates
+  const float* q_err;     // [m] |q - (hi + lo)|
+  const float* db_max2;   // {max |d - (hi + lo)|, max |d|^2} over the valid database rows
+  int n_valid;
+  int* flag_count; int* flag_list;
+};
 int launch_rescore_sort(const float* q, const float* qn, int m, const float* db, const float* dbn, int d,
                         const long long* cand_i, int kc, int k_out, long long idx_base, float* out_dist,
-                        long long* out_idx, cudaStream_t s);
+                        long long* out_idx, const RescoreGuard& guard, cudaStream_t s);
 int launch_pca_finalize(const float* partial, int splits, int N, int P, const float* bias, float* out,
                         cudaStream_t s);
 
@@ -196,8 +230,9 @@ int launch_pca_l2(const float* v, int N, int D, const float* W, const float* b, 
 int launch_l2_normalize_rows(const float* x, int N, int D, float* out, cudaStream_t s);
 int launch_row_sqnorm(const float* x, int N, int D, float* out, cudaStream_t s);
 int launch_scale(const float* x, float s, int n, float* y, cudaStream_t st);
+// err (may be null): |x - (hi + lo)| per row, exact up to the fp32 sum of squares
 int launch_planes_sqnorm(const float* x, int N, int D, __nv_bfloat16* hi, __nv_bfloat16* lo, float* sq,
-                         cudaStream_t st);
+                         cudaStream_t st, float* err = nullptr);
 int launch_l2dist_dense(const float* q, const float* qn, int m, const float* db, const float* dbn,
                         int n, int d, float* out, long long ld_out, cudaStream_t s);
 

@@ -81,7 +81,8 @@ struct ibl_engine {
   DevBuf mrg_d, mrg_i;
   DevBuf bw_g, bw_x, bw_part, bw_w;      // conv backward: dY planes, X planes, wgrad/bias partials, dgrad filter planes
   DevBuf d1_ws;                          // workspace of the single-pass distance/top-k path (tc_dist1.cu)
-  int d1_m = 0, d1_n = 0, d1_d = 0;      // shape of the last call on it (test hook ibl_debug_dist_flagged)
+  DevBuf dguard;                         // guard + exact fallback of the bf16x3 distance/top-k paths
+  const int* dist_flags = nullptr;       // flag counter of the last ibl_l2dist_topk call (null: CUDA-core path)
   DevBuf ssq, nv_part, nv_asum, nvw_pl;  // fused NetVLAD: |x|^2 partials, unit partials, W planes [64,512]
   DevBuf nv_ticket;                      // [images] arrival counters of the fused NetVLAD kernel (zero between launches)
   const float* nvw_pl_src = nullptr;
@@ -273,7 +274,7 @@ int ibl_engine_destroy(ibl_engine* e) {
   DevBuf* bufs[] = {&e->act[0], &e->act[1], &e->feat, &e->nv_assign, &e->nv_inv, &e->nv_raw, &e->vlad,
                     &e->pca_partial, &e->qn, &e->dbn, &e->dist_chunk, &e->cand_d, &e->cand_i,
                     &e->stage_in, &e->stage_out, &e->stage_out2, &e->stage_u8, &e->q_pl, &e->db_pl, &e->v_pl, &e->pca_pl,
-                    &e->mrg_d, &e->mrg_i, &e->d1_ws, &e->bw_g, &e->bw_x, &e->bw_part, &e->bw_w, &e->ssq, &e->nv_part, &e->nv_asum, &e->nvw_pl, &e->nv_ticket};
+                    &e->mrg_d, &e->mrg_i, &e->d1_ws, &e->dguard, &e->bw_g, &e->bw_x, &e->bw_part, &e->bw_w, &e->ssq, &e->nv_part, &e->nv_asum, &e->nvw_pl, &e->nv_ticket};
   for (DevBuf* b : bufs) b->release();
   delete e;
   return IBL_OK;
@@ -944,7 +945,7 @@ int ibl_l2dist_topk(ibl_engine* e, const float* q, int m, const float* db, int n
     // single fp16 tensor-core pass to screen, exact fp32 to decide, guard + exact fallback on the device
     size_t off[9];
     IBL_RET(e->d1_ws.ensure(dist1_workspace_bytes(m, n, d, off)));
-    e->d1_m = m; e->d1_n = n; e->d1_d = d;
+    e->dist_flags = dist1_flag_count(e->d1_ws.p, m, n, d);
     return launch_dist_topk_1pass(q, m, db, n, n_valid, d, k, (long long)idx_base, e->d1_ws.p, out_dist,
                                   reinterpret_cast<long long*>(out_idx), &e->launches, S(stream));
   }
@@ -956,11 +957,33 @@ int ibl_l2dist_topk(ibl_engine* e, const float* q, int m, const float* db, int n
     IBL_RET(e->q_pl.ensure(qe * 4));
     IBL_RET(e->db_pl.ensure(de * 4));
     __nv_bfloat16 *qh = e->q_pl.as<__nv_bfloat16>(), *dh = e->db_pl.as<__nv_bfloat16>();
-    // one pass per matrix: bf16 hi/lo planes for the tensor-core GEMM + exact fp32 squared norms
-    IBL_RET(launch_planes_sqnorm(q, m, d, qh, qh + qe, e->qn.as<float>(), s));
-    IBL_RET(launch_planes_sqnorm(db, n, d, dh, dh + de, e->dbn.as<float>(), s));
-    e->launches += 2;
-    const int kc = 16;                           // candidates kept per query before exact re-scoring
+    // guard workspace: q err [m] | db err [n] | db max2 + flag count (256 B) | flag list [m] | fallback scratch
+    const int kk = k <= 12 ? 16 : (k + 8 > 128 ? 128 : k + 8);   // candidates kept per query before exact re-scoring
+    const size_t g_qe = 0, g_de = g_qe + (((size_t)m * 4 + 255) & ~(size_t)255), g_mx = g_de + (((size_t)n * 4 + 255) & ~(size_t)255);
+    const size_t g_fl = g_mx + 256, g_sc = g_fl + (((size_t)m * 4 + 255) & ~(size_t)255);
+    IBL_RET(e->dguard.ensure(g_sc + dist_exact_scratch_bytes(m, n_valid, k)));
+    uint8_t* gw = reinterpret_cast<uint8_t*>(e->dguard.p);
+    float* q_err = reinterpret_cast<float*>(gw + g_qe);
+    float* db_err = reinterpret_cast<float*>(gw + g_de);
+    RescoreGuard gd{};
+    gd.q_err = q_err; gd.db_max2 = reinterpret_cast<float*>(gw + g_mx); gd.n_valid = n_valid;
+    gd.flag_count = reinterpret_cast<int*>(gw + g_mx + 16); gd.flag_list = reinterpret_cast<int*>(gw + g_fl);
+    e->dist_flags = gd.flag_count;
+    IBL_CUDA_OK(cudaMemsetAsync(gw + g_mx, 0, 32, s));      // db max2 (2 floats) | flag count at +16
+    // one pass per matrix: bf16 hi/lo planes for the tensor-core GEMM + exact fp32 squared norms + the guard's
+    // representation errors
+    IBL_RET(launch_planes_sqnorm(q, m, d, qh, qh + qe, e->qn.as<float>(), s, q_err));
+    IBL_RET(launch_planes_sqnorm(db, n, d, dh, dh + de, e->dbn.as<float>(), s, db_err));
+    IBL_RET(launch_dist_colmax(e->dbn.as<float>(), db_err, 1, n_valid, reinterpret_cast<float*>(gw + g_mx), s));
+    e->launches += 3;
+    // exact brute force of the queries the guard of launch_rescore_sort listed (none, usually)
+    auto fallback = [&]() {
+      e->launches += 2;
+      return launch_dist_exact_fallback(q, e->qn.as<float>(), 1, m, db, e->dbn.as<float>(), 1, n_valid, d, k, idx_base,
+                                        gd.flag_count, gd.flag_list, reinterpret_cast<unsigned long long*>(gw + g_sc),
+                                        out_dist, reinterpret_cast<long long*>(out_idx), s);
+    };
+    const int kc = 16;
     if (k <= 12) {
       // SM pairs (tcgen05.mma.cta_group::2, tc_gemm2.cu) unless there is a single 128-query tile; IBL_DIST_2SM=0
       // selects the one-SM kernel of tc_gemm.cu
@@ -980,6 +1003,7 @@ int ibl_l2dist_topk(ibl_engine* e, const float* q, int m, const float* db, int n
       }
       e->launches++;
       const long long* ci = e->cand_i.as<long long>();
+      gd.cand_sd = e->cand_d.as<float>();
       if (runs > 1) {
         IBL_RET(e->mrg_d.ensure((size_t)m * kc * sizeof(float)));
         IBL_RET(e->mrg_i.ensure((size_t)m * kc * sizeof(int64_t)));
@@ -987,16 +1011,17 @@ int ibl_l2dist_topk(ibl_engine* e, const float* q, int m, const float* db, int n
                                   e->mrg_d.as<float>(), e->mrg_i.as<int64_t>(), s));
         e->launches++;
         ci = e->mrg_i.as<long long>();
+        gd.cand_sd = e->mrg_d.as<float>();
       }
       IBL_RET(launch_rescore_sort(q, e->qn.as<float>(), m, db, e->dbn.as<float>(), d, ci, kc, k, idx_base,
-                                  out_dist, reinterpret_cast<long long*>(out_idx), s));
+                                  out_dist, reinterpret_cast<long long*>(out_idx), gd, s));
       e->launches++;
-      return IBL_OK;
+      return fallback();
     }
-    // k > 12: dense tiles on the tensor cores, row select, then the same exact re-scoring
+    // k > 12: dense tiles on the tensor cores, row select, then the same exact re-scoring.  k >= 121 keeps fewer than
+    // 8 candidates beyond the k-th: expect the guard to send most such queries to the exact brute force.
     const int CHT = 32768;
     const int ncht = cdiv(n_valid, CHT);
-    const int kk = k + 8 > 128 ? 128 : k + 8;
     IBL_REQUIRE((long long)ncht * kk <= 8192, "database shard too large for one call; shard it");
     const int chw = n_valid < CHT ? cdiv(n_valid, 4) * 4 : CHT;
     IBL_RET(e->dist_chunk.ensure((size_t)m * chw * sizeof(float)));
@@ -1012,6 +1037,7 @@ int ibl_l2dist_topk(ibl_engine* e, const float* q, int m, const float* db, int n
       e->launches += 2;
     }
     const long long* ci = e->cand_i.as<long long>();
+    gd.cand_sd = e->cand_d.as<float>();
     if (ncht > 1) {
       IBL_RET(e->mrg_d.ensure((size_t)m * kk * sizeof(float)));
       IBL_RET(e->mrg_i.ensure((size_t)m * kk * sizeof(int64_t)));
@@ -1019,12 +1045,14 @@ int ibl_l2dist_topk(ibl_engine* e, const float* q, int m, const float* db, int n
                                 e->mrg_d.as<float>(), e->mrg_i.as<int64_t>(), s));
       e->launches++;
       ci = e->mrg_i.as<long long>();
+      gd.cand_sd = e->mrg_d.as<float>();
     }
     IBL_RET(launch_rescore_sort(q, e->qn.as<float>(), m, db, e->dbn.as<float>(), d, ci, kk, k, idx_base, out_dist,
-                                reinterpret_cast<long long*>(out_idx), s));
+                                reinterpret_cast<long long*>(out_idx), gd, s));
     e->launches++;
-    return IBL_OK;
+    return fallback();
   }
+  e->dist_flags = nullptr;
   const int CH = 32768;                         // database rows per dense chunk
   const int nch = n_valid > 0 ? cdiv(n_valid, CH) : 1;
   IBL_REQUIRE((long long)nch * k <= 8192, "database shard too large for one call; shard it");
@@ -1112,14 +1140,16 @@ int ibl_l2dist_topk_host(ibl_engine* e, const float* q_host, int m, const float*
   return IBL_OK;
 }
 
-// test hook: how many queries the guard of the single-pass distance path listed in the last ibl_l2dist_topk call
-// (they were re-ranked by exact brute force on the device).  Synchronises the stream.
+// test hook: how many queries the screening guard listed in the last ibl_l2dist_topk call (they were re-ranked by
+// exact brute force on the device), whichever tensor-core path it took; -1 after the CUDA-core path.  Synchronises.
 int ibl_debug_dist_flagged(ibl_engine* e, int* count, void* stream) {
   IBL_REQUIRE(e && count, "null argument");
   *count = -1;
-  if (!e->d1_ws.p || !e->d1_m) return IBL_OK;
+  if (!e->dist_flags) return IBL_OK;
   DeviceGuard g(e->device);
-  return dist1_last_flag_count(e->d1_ws.p, e->d1_m, e->d1_n, e->d1_d, count, S(stream));
+  IBL_CUDA_OK(cudaMemcpyAsync(count, e->dist_flags, sizeof(int), cudaMemcpyDeviceToHost, S(stream)));
+  IBL_CUDA_OK(cudaStreamSynchronize(S(stream)));
+  return IBL_OK;
 }
 
 int ibl_selftest_tc(ibl_engine* e, float* max_rel_err) {

@@ -258,42 +258,53 @@ int launch_scale(const float* x, float s, int n, float* y, cudaStream_t st) {
 
 namespace ibl {
 // One pass over a row-major fp32 matrix: bf16 hi/lo planes + squared row norms (what the distance GEMM and
-// its epilogue need), instead of separate f32_to_planes and row_sqnorm passes.  One block per row.
+// its epilogue need), instead of separate f32_to_planes and row_sqnorm passes.  One block per row.  err (may be
+// null): |x - (hi + lo)| of the row, for the screening guard; x - hi and (x - hi) - lo are exact in fp32.
 __global__ void __launch_bounds__(256)
 planes_sqnorm_kernel(const float* __restrict__ x, int D, __nv_bfloat16* __restrict__ hi,
-                     __nv_bfloat16* __restrict__ lo, float* __restrict__ sq) {
-  __shared__ float red[8];
+                     __nv_bfloat16* __restrict__ lo, float* __restrict__ sq, float* __restrict__ err) {
+  __shared__ float red[8], rede[8];
   const long long r = blockIdx.x;
   const float4* p = reinterpret_cast<const float4*>(x + r * D);
   uint2* ph = reinterpret_cast<uint2*>(hi + r * D);
   uint2* pl = reinterpret_cast<uint2*>(lo + r * D);
-  float ss = 0.f;
+  float ss = 0.f, se = 0.f;
   for (int i = threadIdx.x; i < D / 4; i += blockDim.x) {
     const float4 v = __ldg(p + i);
     ss = fmaf(v.x, v.x, ss); ss = fmaf(v.y, v.y, ss); ss = fmaf(v.z, v.z, ss); ss = fmaf(v.w, v.w, ss);
     const __nv_bfloat16 h0 = __float2bfloat16_rn(v.x), h1 = __float2bfloat16_rn(v.y);
     const __nv_bfloat16 h2 = __float2bfloat16_rn(v.z), h3 = __float2bfloat16_rn(v.w);
     __nv_bfloat162 a(h0, h1), b(h2, h3);
-    __nv_bfloat162 c = __floats2bfloat162_rn(v.x - __bfloat162float(h0), v.y - __bfloat162float(h1));
-    __nv_bfloat162 d = __floats2bfloat162_rn(v.z - __bfloat162float(h2), v.w - __bfloat162float(h3));
+    const float r0 = v.x - __bfloat162float(h0), r1 = v.y - __bfloat162float(h1);
+    const float r2 = v.z - __bfloat162float(h2), r3 = v.w - __bfloat162float(h3);
+    __nv_bfloat162 c = __floats2bfloat162_rn(r0, r1);
+    __nv_bfloat162 d = __floats2bfloat162_rn(r2, r3);
+    if (err) {
+      const float e0 = r0 - __low2float(c), e1 = r1 - __high2float(c), e2 = r2 - __low2float(d), e3 = r3 - __high2float(d);
+      se = fmaf(e0, e0, se); se = fmaf(e1, e1, se); se = fmaf(e2, e2, se); se = fmaf(e3, e3, se);
+    }
     ph[i] = make_uint2(*reinterpret_cast<uint32_t*>(&a), *reinterpret_cast<uint32_t*>(&b));
     pl[i] = make_uint2(*reinterpret_cast<uint32_t*>(&c), *reinterpret_cast<uint32_t*>(&d));
   }
 #pragma unroll
-  for (int o = 16; o > 0; o >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, o);
-  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = ss;
+  for (int o = 16; o > 0; o >>= 1) {
+    ss += __shfl_xor_sync(0xffffffffu, ss, o);
+    se += __shfl_xor_sync(0xffffffffu, se, o);
+  }
+  if ((threadIdx.x & 31) == 0) { red[threadIdx.x >> 5] = ss; rede[threadIdx.x >> 5] = se; }
   __syncthreads();
   if (threadIdx.x == 0) {
-    float tot = 0.f;
-    for (int i = 0; i < (int)(blockDim.x >> 5); ++i) tot += red[i];
+    float tot = 0.f, tote = 0.f;
+    for (int i = 0; i < (int)(blockDim.x >> 5); ++i) { tot += red[i]; tote += rede[i]; }
     sq[r] = tot;
+    if (err) err[r] = sqrtf(tote);
   }
 }
 int launch_planes_sqnorm(const float* x, int N, int D, __nv_bfloat16* hi, __nv_bfloat16* lo, float* sq,
-                         cudaStream_t st) {
+                         cudaStream_t st, float* err) {
   IBL_REQUIRE(D % 4 == 0, "planes_sqnorm: D must be a multiple of 4");
   if (N <= 0) return IBL_OK;
-  planes_sqnorm_kernel<<<N, 256, 0, st>>>(x, D, hi, lo, sq);
+  planes_sqnorm_kernel<<<N, 256, 0, st>>>(x, D, hi, lo, sq, err);
   IBL_CUDA_OK(cudaGetLastError());
   return IBL_OK;
 }

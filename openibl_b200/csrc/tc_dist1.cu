@@ -5,8 +5,8 @@
 // fp32 anyway.  Here:
 //   1. rows_f16_kernel        one pass per matrix: fp16 plane of each row scaled by a power of two (row max in
 //                             [0.5,1): no overflow, 11 significant bits), exact fp32 |x|^2 (same summation order as
-//                             planes_sqnorm_kernel, so the exact distances below are unchanged), the 4-norm and
-//                             the max of each row (error model of the guard);
+//                             planes_sqnorm_kernel, so the exact distances below are unchanged) and the row's
+//                             representation error |x - plane * 2^e| (exact per element, fp16 subnormals included);
 //   2. gemm2_f16_top16_kernel tcgen05.mma.cta_group::2 kind::f16 (fp16 x fp16 -> fp32 in TMEM), ONE MMA per
 //                             K step, 256 queries x 256 database rows per SM pair, 6-stage TMA ring, running
 //                             top-16 per query in registers across the pair's database range;
@@ -14,12 +14,15 @@
 //                             survivors (|q|^2 + |d|^2 - 2 q.d, bit-identical to round 1's rescore_sort_kernel),
 //                             final (dist, idx) sort, and the GUARD: a database row that was NOT kept has a
 //                             screened distance >= s16 (the 16th screened distance); its exact distance is
-//                             >= s16 - B, B = 8 sigma of the fp16 rounding error of one dot product (from the rows'
-//                             4-norms) + the absolute error of fp16 subnormals.  If s16 - B < (k-th exact distance)
-//                             the query is appended to a device-side list;
-//   4. dist_exact_chunk_kernel / dist_exact_merge_kernel   listed queries (none, in practice: the k-th to 16th gap
-//                             is ~50 B for descriptor-like data) are ranked again by exact fp32 brute force,
-//                             without any host round trip: the kernels size their work from the device counter.
+//                             >= s16 - B with B = screen_guard_bound (common.cuh), a bound for any input: the
+//                             representation errors of the query and of the worst database row (Cauchy-Schwarz),
+//                             the TMEM accumulator's truncation (d/16 MMAs, per-MMA loss from the kind::bf16
+//                             measurement x 18) and fp32 rounding of both distance expressions.  Unless
+//                             s16 - B > (k-th exact distance) the query is appended to a device-side list;
+//   4. dist_exact_chunk_kernel / dist_exact_merge_kernel   listed queries (none on descriptor-like data: B is
+//                             ~8e-4 for unit 4096-d rows, the k-th to 16th gap is larger) are ranked again by exact
+//                             fp32 brute force, without any host round trip: the kernels size their work from the
+//                             device counter.  The bf16x3 paths of ibl_l2dist_topk use the same fallback.
 #include <cuda_fp16.h>
 #include <stdlib.h>
 
@@ -31,68 +34,84 @@ namespace ibl {
 using namespace tc;
 
 // ---- 1. fp16 planes -----------------------------------------------------------------------------
-// aux[r] = {|x|^2 (exact fp32), 2^e (x = plane * 2^e), (sum x^4)^(1/4), max|x|}
+// aux[r] = {|x|^2 (exact fp32), 2^e (x = plane * 2^e), |x - plane * 2^e|, 0}
 __global__ void __launch_bounds__(256)
 rows_f16_kernel(const float* __restrict__ x, int D, __half* __restrict__ plane, float4* __restrict__ aux) {
-  __shared__ float red[8], red4[8], redm[8];
-  __shared__ float scale_s;
+  __shared__ float red[8], redm[8];
+  __shared__ float scale_s, tot_s;
   const long long r = blockIdx.x;
   const float4* p = reinterpret_cast<const float4*>(x + r * D);
-  float ss = 0.f, s4 = 0.f, mx = 0.f;
+  float ss = 0.f, mx = 0.f;
   for (int i = threadIdx.x; i < D / 4; i += blockDim.x) {
     const float4 v = __ldg(p + i);
     ss = fmaf(v.x, v.x, ss); ss = fmaf(v.y, v.y, ss); ss = fmaf(v.z, v.z, ss); ss = fmaf(v.w, v.w, ss);
-    const float a = v.x * v.x, b = v.y * v.y, c = v.z * v.z, d = v.w * v.w;
-    s4 = fmaf(a, a, s4); s4 = fmaf(b, b, s4); s4 = fmaf(c, c, s4); s4 = fmaf(d, d, s4);
     mx = fmaxf(fmaxf(mx, fmaxf(fabsf(v.x), fabsf(v.y))), fmaxf(fabsf(v.z), fabsf(v.w)));
   }
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) {
     ss += __shfl_xor_sync(0xffffffffu, ss, o);
-    s4 += __shfl_xor_sync(0xffffffffu, s4, o);
     mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
   }
-  if ((threadIdx.x & 31) == 0) { red[threadIdx.x >> 5] = ss; red4[threadIdx.x >> 5] = s4; redm[threadIdx.x >> 5] = mx; }
+  if ((threadIdx.x & 31) == 0) { red[threadIdx.x >> 5] = ss; redm[threadIdx.x >> 5] = mx; }
   __syncthreads();
   if (threadIdx.x == 0) {
-    float tot = 0.f, tot4 = 0.f, m = 0.f;
-    for (int i = 0; i < (int)(blockDim.x >> 5); ++i) { tot += red[i]; tot4 += red4[i]; m = fmaxf(m, redm[i]); }
+    float tot = 0.f, m = 0.f;
+    for (int i = 0; i < (int)(blockDim.x >> 5); ++i) { tot += red[i]; m = fmaxf(m, redm[i]); }
     int e = 0;
     if (m > 0.f && m < INFINITY) frexpf(m, &e);       // m = f * 2^e, f in [0.5, 1)
-    const float sc = ldexpf(1.f, e);
     scale_s = ldexpf(1.f, -e);
-    aux[r] = make_float4(tot, sc, sqrtf(sqrtf(tot4)), m);
+    tot_s = tot;
   }
   __syncthreads();
-  const float inv = scale_s;
+  const float inv = scale_s, sc = 1.f / inv;
   uint2* ph = reinterpret_cast<uint2*>(plane + r * D);
+  float se = 0.f;
   for (int i = threadIdx.x; i < D / 4; i += blockDim.x) {   // second read of the row: L1/L2 hits
     const float4 v = __ldg(p + i);
     const __half2 a = __floats2half2_rn(v.x * inv, v.y * inv), b = __floats2half2_rn(v.z * inv, v.w * inv);
     ph[i] = make_uint2(*reinterpret_cast<const uint32_t*>(&a), *reinterpret_cast<const uint32_t*>(&b));
+    // x - plane * 2^e: the product is exact and the difference is exact (Sterbenz; or plane = 0)
+    const float e0 = v.x - __low2float(a) * sc, e1 = v.y - __high2float(a) * sc;
+    const float e2 = v.z - __low2float(b) * sc, e3 = v.w - __high2float(b) * sc;
+    se = fmaf(e0, e0, se); se = fmaf(e1, e1, se); se = fmaf(e2, e2, se); se = fmaf(e3, e3, se);
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) se += __shfl_xor_sync(0xffffffffu, se, o);
+  __syncthreads();                                     // red[] of the first reduction has been read
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = se;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    float tote = 0.f;
+    for (int i = 0; i < (int)(blockDim.x >> 5); ++i) tote += red[i];
+    aux[r] = make_float4(tot_s, sc, sqrtf(tote), 0.f);
   }
 }
 
-// max over the database rows of (4-norm, max|x|, |x|^2): the guard's bound for rows that were not kept
-__global__ void dist_colmax_kernel(const float4* __restrict__ aux, int n, float* __restrict__ out3) {
-  float a = 0.f, b = 0.f, c = 0.f;
+// max over the database rows of (|x - x'|, |x|^2): the guard's bound for rows that were not kept.  sq / err are
+// read with a stride (4: the float4 aux of this file; 1: plain arrays of the bf16x3 path).
+__global__ void dist_colmax_kernel(const float* __restrict__ sq, const float* __restrict__ err, int stride, int n,
+                                   float* __restrict__ out2) {
+  float a = 0.f, c = 0.f;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-    const float4 v = __ldg(aux + i);
-    a = fmaxf(a, v.z);
-    b = fmaxf(b, v.w);
-    c = fmaxf(c, v.x);
+    a = fmaxf(a, __ldg(err + (long long)i * stride));
+    c = fmaxf(c, __ldg(sq + (long long)i * stride));
   }
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) {
     a = fmaxf(a, __shfl_xor_sync(0xffffffffu, a, o));
-    b = fmaxf(b, __shfl_xor_sync(0xffffffffu, b, o));
     c = fmaxf(c, __shfl_xor_sync(0xffffffffu, c, o));
   }
   if ((threadIdx.x & 31) == 0) {     // non-negative floats order like their bit patterns
-    atomicMax(reinterpret_cast<int*>(out3), __float_as_int(a));
-    atomicMax(reinterpret_cast<int*>(out3) + 1, __float_as_int(b));
-    atomicMax(reinterpret_cast<int*>(out3) + 2, __float_as_int(c));
+    atomicMax(reinterpret_cast<int*>(out2), __float_as_int(a));
+    atomicMax(reinterpret_cast<int*>(out2) + 1, __float_as_int(c));
   }
+}
+
+int launch_dist_colmax(const float* sq, const float* err, int stride, int n, float* out2, cudaStream_t s) {
+  if (n <= 0) return IBL_OK;
+  dist_colmax_kernel<<<cdiv(n, 256) < 64 ? cdiv(n, 256) : 64, 256, 0, s>>>(sq, err, stride, n, out2);
+  IBL_CUDA_OK(cudaGetLastError());
+  return IBL_OK;
 }
 
 // ---- 2. screening GEMM on SM pairs ----------------------------------------------------------------
@@ -423,7 +442,8 @@ gemm2_f16_top16_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_co
 __device__ __forceinline__ float d1_exact(const float* qrow, const float* __restrict__ dp, int d, int lane, float an,
                                           float bn) {
   float acc = 0.f;
-  for (int i = lane * 4; i < d; i += 128) {
+#pragma unroll 2
+  for (int i = lane * 4; i < d; i += 128) {   // unrolled: several row loads in flight (the FMA order is unchanged)
     const float4 a = *reinterpret_cast<const float4*>(qrow + i);
     const float4 b = __ldg(reinterpret_cast<const float4*>(dp + i));
     acc = fmaf(a.x, b.x, acc); acc = fmaf(a.y, b.y, acc);
@@ -437,17 +457,13 @@ __device__ __forceinline__ float d1_exact(const float* qrow, const float* __rest
 struct FinishArgs {
   const float* q; const float* db;
   const float4* q_aux; const float4* db_aux;
-  const float* db_max2;          // {max 4-norm, max |x|, max |x|^2} over the database rows
+  const float* db_max2;          // {max |x - x'|, max |x|^2} over the database rows
   const float* cand_d; const int* cand_i;
   int m, d, runs, k_out, n_valid;
   long long idx_base;
   float* out_dist; long long* out_idx;
   int* flag_count; int* flag_list;
 };
-
-// kappa = 8 standard deviations; rms relative rounding error of fp16 RN = 2^-11 * 0.41; two operands (sqrt 2);
-// distance = -2 dot (factor 2)  ->  8 * 2 * 1.414 * 0.41 * 2^-11
-#define D1_GUARD_C (8.f * 2.f * 1.41421356f * 0.41f * 4.8828125e-4f)
 
 __global__ void __launch_bounds__(128)
 dist_finish_kernel(const FinishArgs g) {
@@ -535,12 +551,7 @@ dist_finish_kernel(const FinishArgs g) {
     bool flag = (s16k == ~0ull) || (ek == ~0ull);        // cannot happen with n_valid > 16; be safe
     if (!flag) {
       const float s16 = d1_unord((uint32_t)(s16k >> 32)), e_k = d1_unord((uint32_t)(ek >> 32));
-      // statistical part: 8 sigma of the fp16 rounding error of one dot product (Cauchy-Schwarz on the 4-norms);
-      // absolute part: values below 2^-14 of the row max are fp16 subnormals, error <= 2^-24 * row max each:
-      // |dot error| <= 2^-24 sqrt(D) (dmax |q| + qmax |d|), distance = -2 dot
-      const float bound = D1_GUARD_C * qa.z * __ldg(g.db_max2) +
-                          2.f * 5.9604645e-8f * sqrtf((float)d) *
-                              (__ldg(g.db_max2 + 1) * sqrtf(qa.x) + qa.w * sqrtf(__ldg(g.db_max2 + 2)));
+      const float bound = screen_guard_bound(qa.x, qa.z, __ldg(g.db_max2 + 1), __ldg(g.db_max2), d, d / 16, 0.f);
       flag = !(s16 - bound > e_k);                       // also catches NaN
     }
     if (flag) g.flag_list[atomicAdd(g.flag_count, 1)] = (int)row;
@@ -548,98 +559,198 @@ dist_finish_kernel(const FinishArgs g) {
 }
 
 // ---- 4. exact brute force for the listed queries ----------------------------------------------------
-constexpr int DX_CHUNK = 4096;    // database rows per work item
+constexpr int DX_KMAX = 128;
+constexpr int DX_G = 8;                 // listed queries per work item of the exact brute force
+constexpr int DX_QSTAGE = 32768;        // floats of staged queries per work item (128 KiB)
+// database rows per work item: at most 64 items per listed query (bounds the scratch), at least 128 rows, so that a
+// few listed queries still spread over all SMs (each warp's rows are a chain of L2 latencies)
+static int dx_chunk_rows(int n_valid) {
+  const int c = cdiv(cdiv(n_valid > 0 ? n_valid : 1, 64), 64) * 64;
+  return c > 128 ? c : 128;
+}
 
 struct ExactArgs {
   const float* q; const float* db;
-  const float4* q_aux; const float4* db_aux;
-  int m, d, n_valid, k, nchunks;
+  const float* qn; const float* dbn;   // |x|^2, read with a stride (4 for the float4 aux of this file)
+  int qn_stride, dbn_stride;
+  int m, d, n_valid, k, chunk, nchunks, group;
   long long idx_base;
   const int* flag_count; const int* flag_list;
-  unsigned long long* scratch;   // [m][nchunks][16] keys
+  unsigned long long* scratch;   // [m][nchunks][k] keys
   float* out_dist; long long* out_idx;
 };
 
-// work item = (listed query f, chunk c): exact distances of DX_CHUNK rows, the 16 smallest keys to scratch
+// number of keys below `key` in nl sorted lists of length k (stride k); keys are distinct (they hold the row)
+__device__ __forceinline__ int dx_rank(const unsigned long long* lists, int nl, int k, unsigned long long key) {
+  int rank = 0;
+  for (int l = 0; l < nl && rank < k; ++l) {
+    const unsigned long long* L = lists + (long long)l * k;
+    int lo = 0, hi = k;
+    while (lo < hi) { const int mid = (lo + hi) >> 1; if (L[mid] < key) lo = mid + 1; else hi = mid; }
+    rank += lo;
+  }
+  return rank;
+}
+
+// work item = (chunk c of the database, group of up to g.group listed queries): every database row of the chunk is read
+// once for the whole group (one warp per row, the group's queries staged in shared memory), so a handful of listed
+// queries costs about one pass over the database.  Per query and warp a sorted list of the k best keys; at the end of
+// the item the 8 lists of each query are merged by rank into scratch.  The dot products use d1_exact's arithmetic
+// (lane-strided FMAs in the same order, the same xor tree), so the distances are bit-identical to the re-scoring.
 __global__ void __launch_bounds__(256)
 dist_exact_chunk_kernel(const ExactArgs g) {
-  extern __shared__ __align__(16) float qs[];
-  __shared__ unsigned long long best[8][16];
+  extern __shared__ __align__(16) float dsm[];   // [group][d] queries when staged | [group][8 warps][k] keys
+  const int G = g.group, k = g.k, d = g.d;
+  const bool staged = (long long)G * d <= DX_QSTAGE;
+  unsigned long long* lists = reinterpret_cast<unsigned long long*>(dsm + (staged ? G * d : 0));
   const int count = *g.flag_count;
-  const int items = count * g.nchunks;
+  const int ngroups = (count + G - 1) / G;
+  const int items = ngroups * g.nchunks;
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  const bool staged = g.d <= 16384;
   for (int item = blockIdx.x; item < items; item += gridDim.x) {
-    const int f = item / g.nchunks, c = item - f * g.nchunks;
-    const long long row = g.flag_list[f];
+    const int c = item / ngroups, grp = item - c * ngroups;   // the groups of one chunk run side by side: L2 hits
+    const int f0 = grp * G, gn = min(G, count - f0);
     __syncthreads();
     if (staged)
-      for (int i = threadIdx.x * 4; i < g.d; i += 256 * 4)
-        *reinterpret_cast<float4*>(qs + i) = __ldg(reinterpret_cast<const float4*>(g.q + row * g.d + i));
+      for (int t = 0; t < gn; ++t) {
+        const long long row = g.flag_list[f0 + t];
+        for (int i = threadIdx.x * 4; i < d; i += 256 * 4)
+          *reinterpret_cast<float4*>(dsm + t * d + i) = __ldg(reinterpret_cast<const float4*>(g.q + row * d + i));
+      }
+    for (int s = threadIdx.x; s < G * 8 * k; s += 256) lists[s] = ~0ull;
     __syncthreads();
-    const float* qrow = staged ? qs : (g.q + row * g.d);
-    const float an = __ldg(&g.q_aux[row].x);
-    unsigned long long mine[16];               // this warp's 16 best (every lane holds the same list)
+    const float* qp[DX_G];
+    float an[DX_G];
 #pragma unroll
-    for (int j = 0; j < 16; ++j) mine[j] = ~0ull;
-    const int j0 = c * DX_CHUNK, j1 = min(g.n_valid, j0 + DX_CHUNK);
+    for (int t = 0; t < DX_G; ++t) {
+      const long long row = t < gn ? g.flag_list[f0 + t] : 0;
+      qp[t] = staged ? dsm + t * d : g.q + row * d;
+      an[t] = t < gn ? __ldg(g.qn + row * g.qn_stride) : 0.f;
+    }
+    const int j0 = c * g.chunk, j1 = min(g.n_valid, j0 + g.chunk);
     for (int j = j0 + wid; j < j1; j += 8) {
-      const float dist = d1_exact(qrow, g.db + (long long)j * g.d, g.d, lane, an, __ldg(&g.db_aux[j].x));
-      unsigned long long key = ((unsigned long long)d1_ord(dist) << 32) | (unsigned)j;
-      if (key < mine[15]) {
-        mine[15] = key;
+      const float* dp = g.db + (long long)j * d;
+      float acc[DX_G];
 #pragma unroll
-        for (int s = 15; s > 0; --s)
-          if (mine[s] < mine[s - 1]) { const unsigned long long t = mine[s]; mine[s] = mine[s - 1]; mine[s - 1] = t; }
+      for (int t = 0; t < DX_G; ++t) acc[t] = 0.f;
+#pragma unroll 2
+      for (int i = lane * 4; i < d; i += 128) {
+        const float4 b = __ldg(reinterpret_cast<const float4*>(dp + i));
+#pragma unroll
+        for (int t = 0; t < DX_G; ++t) {
+          if (t < gn) {
+            const float4 a = *reinterpret_cast<const float4*>(qp[t] + i);
+            acc[t] = fmaf(a.x, b.x, acc[t]); acc[t] = fmaf(a.y, b.y, acc[t]);
+            acc[t] = fmaf(a.z, b.z, acc[t]); acc[t] = fmaf(a.w, b.w, acc[t]);
+          }
+        }
+      }
+      const float bn = __ldg(g.dbn + (long long)j * g.dbn_stride);
+#pragma unroll
+      for (int t = 0; t < DX_G; ++t) {
+        if (t >= gn) break;
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) acc[t] += __shfl_xor_sync(0xffffffffu, acc[t], o);
+        const float dist = fmaf(-2.f, acc[t], an[t] + bn);
+        const unsigned long long key = ((unsigned long long)d1_ord(dist) << 32) | (unsigned)j;
+        unsigned long long* L = lists + (t * 8 + wid) * k;
+        if (key < L[k - 1]) {                  // warp-uniform: sorted insert, each lane moves the slots it owns
+          unsigned long long left[DX_KMAX / 32], cur[DX_KMAX / 32];
+#pragma unroll
+          for (int u = 0; u < DX_KMAX / 32; ++u) {
+            const int s = lane + 32 * u;
+            left[u] = (s > 0 && s < k) ? L[s - 1] : 0ull;
+            cur[u] = s < k ? L[s] : 0ull;
+          }
+          __syncwarp();
+#pragma unroll
+          for (int u = 0; u < DX_KMAX / 32; ++u) {
+            const int s = lane + 32 * u;
+            if (s < k) {
+              if (s > 0 && left[u] > key) L[s] = left[u];
+              else if (cur[u] > key) L[s] = key;
+            }
+          }
+          __syncwarp();
+        }
       }
     }
-    if (lane == 0)
-#pragma unroll
-      for (int j = 0; j < 16; ++j) best[wid][j] = mine[j];
     __syncthreads();
-    if (threadIdx.x == 0) {                    // 16 smallest of the 8 sorted lists (rare path: serial merge)
-      int head[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-      unsigned long long* out = g.scratch + ((long long)row * g.nchunks + c) * 16;
-      for (int t = 0; t < 16; ++t) {
-        int bw = 0;
-        unsigned long long bk = ~0ull;
-        for (int w = 0; w < 8; ++w)
-          if (head[w] < 16 && best[w][head[w]] < bk) { bk = best[w][head[w]]; bw = w; }
-        out[t] = bk;
-        if (bk != ~0ull) ++head[bw];
-      }
+    // per query: the k smallest of its 8 sorted lists, placed by rank
+    for (int t = 0; t < gn; ++t) {
+      const long long row = g.flag_list[f0 + t];
+      unsigned long long* out = g.scratch + ((long long)row * g.nchunks + c) * k;
+      for (int s = threadIdx.x; s < k; s += 256) out[s] = ~0ull;
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < gn * 8 * k; i += 256) {
+      const unsigned long long key = lists[i];
+      if (key == ~0ull) continue;
+      const int t = i / (8 * k);
+      const int rank = dx_rank(lists + t * 8 * k, 8, k, key);
+      if (rank < k) g.scratch[((long long)g.flag_list[f0 + t] * g.nchunks + c) * k + rank] = key;
     }
   }
 }
 
-// one block per listed query: merge its nchunks x 16 keys, write the final top-k over the guarded result
+// one block per listed query: the k smallest of its nchunks sorted lists (staged in shared memory), placed by rank
 __global__ void __launch_bounds__(128)
 dist_exact_merge_kernel(const ExactArgs g) {
+  extern __shared__ unsigned long long src[];   // [nchunks][k]
   const int count = *g.flag_count;
   for (int f = blockIdx.x; f < count; f += gridDim.x) {
     const long long row = g.flag_list[f];
-    const unsigned long long* src = g.scratch + row * g.nchunks * 16;
-    if (threadIdx.x == 0) {                    // rare path: a serial k-way selection is fine
-      unsigned long long prev = 0;
-      bool first = true;
-      for (int t = 0; t < g.k; ++t) {
-        unsigned long long bk = ~0ull;
-        for (int i = 0; i < g.nchunks * 16; ++i) {
-          const unsigned long long key = src[i];
-          if ((first || key > prev) && key < bk) bk = key;
-        }
-        if (bk == ~0ull) {
-          g.out_dist[row * g.k + t] = INFINITY;
-          g.out_idx[row * g.k + t] = -1;
-        } else {
-          g.out_dist[row * g.k + t] = d1_unord((uint32_t)(bk >> 32));
-          g.out_idx[row * g.k + t] = g.idx_base + (long long)(uint32_t)(bk & 0xffffffffu);
-        }
-        prev = bk;
-        first = false;
+    __syncthreads();
+    for (int i = threadIdx.x; i < g.nchunks * g.k; i += blockDim.x) src[i] = g.scratch[row * g.nchunks * g.k + i];
+    for (int t = threadIdx.x; t < g.k; t += blockDim.x) {
+      g.out_dist[row * g.k + t] = INFINITY;
+      g.out_idx[row * g.k + t] = -1;
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < g.nchunks * g.k; i += blockDim.x) {
+      const unsigned long long key = src[i];
+      if (key == ~0ull) continue;
+      const int rank = dx_rank(src, g.nchunks, g.k, key);
+      if (rank < g.k) {
+        g.out_dist[row * g.k + rank] = d1_unord((uint32_t)(key >> 32));
+        g.out_idx[row * g.k + rank] = g.idx_base + (long long)(uint32_t)(key & 0xffffffffu);
       }
     }
+    __syncthreads();
   }
+}
+
+size_t dist_exact_scratch_bytes(int m, int n_valid, int k) {
+  const int nchunks = cdiv(n_valid > 0 ? n_valid : 1, 128);    // >= the chunks of any n_valid' <= n_valid
+  return (size_t)m * (nchunks < 64 ? nchunks : 64) * k * sizeof(unsigned long long);
+}
+
+// exact fp32 brute force of the queries in flag_list[0 .. *flag_count): no host round trip, the kernels size their
+// work from the device counter and exit at once when nothing is listed.  scratch: dist_exact_scratch_bytes(m, n_valid, k)
+int launch_dist_exact_fallback(const float* q, const float* qn, int qn_stride, int m, const float* db, const float* dbn,
+                               int dbn_stride, int n_valid, int d, int k, long long idx_base, const int* flag_count,
+                               const int* flag_list, unsigned long long* scratch, float* out_dist, long long* out_idx,
+                               cudaStream_t s) {
+  IBL_REQUIRE(k >= 1 && k <= DX_KMAX && d % 4 == 0, "exact fallback: 1 <= k <= 128, d % 4 == 0");
+  static DeviceOnce attr_done;   // the attribute is per device
+  if (!attr_done.done()) {
+    IBL_CUDA_OK(cudaFuncSetAttribute(dist_exact_chunk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                     DX_QSTAGE * 4 + DX_G * 8 * DX_KMAX * 8));
+    IBL_CUDA_OK(cudaFuncSetAttribute(dist_exact_merge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
+    attr_done.mark();
+  }
+  ExactArgs x{};
+  x.q = q; x.db = db; x.qn = qn; x.dbn = dbn; x.qn_stride = qn_stride; x.dbn_stride = dbn_stride;
+  x.m = m; x.d = d; x.n_valid = n_valid; x.k = k;
+  x.group = d <= DX_QSTAGE / DX_G ? DX_G : (d <= DX_QSTAGE ? DX_QSTAGE / d : 1);
+  x.chunk = dx_chunk_rows(n_valid);
+  x.nchunks = cdiv(n_valid > 0 ? n_valid : 1, x.chunk); x.idx_base = idx_base; x.flag_count = flag_count;
+  x.flag_list = flag_list; x.scratch = scratch; x.out_dist = out_dist; x.out_idx = out_idx;
+  const size_t csm = ((long long)x.group * d <= DX_QSTAGE ? (size_t)x.group * d * 4 : 0) + (size_t)x.group * 8 * k * 8;
+  dist_exact_chunk_kernel<<<device_sm_count() * 2, 256, csm, s>>>(x);
+  dist_exact_merge_kernel<<<128, 128, (size_t)x.nchunks * k * sizeof(unsigned long long), s>>>(x);
+  IBL_CUDA_OK(cudaGetLastError());
+  return IBL_OK;
 }
 
 // ---- host -----------------------------------------------------------------------------------------
@@ -668,8 +779,7 @@ size_t dist1_workspace_bytes(int m, int n, int d, size_t* off /*[8]*/) {
   off[5] = take((size_t)m * 4 + (size_t)m * 4);     // guard list | shared gates
   off[6] = take((size_t)8 * m * 16 * 4);
   off[7] = take((size_t)8 * m * 16 * 4);
-  const int nchunks = cdiv(n > 0 ? n : 1, DX_CHUNK);
-  off[8] = take((size_t)m * nchunks * 16 * 8);
+  off[8] = take(dist_exact_scratch_bytes(m, n, 16));
   return o;
 }
 
@@ -692,12 +802,12 @@ int launch_dist_topk_1pass(const float* q, int m, const float* db, int n, int n_
   int* ci = reinterpret_cast<int*>(w + off[7]);
   unsigned long long* scratch = reinterpret_cast<unsigned long long*>(w + off[8]);
 
-  IBL_CUDA_OK(cudaMemsetAsync(w + off[4], 0, 32, s));
+  IBL_CUDA_OK(cudaMemsetAsync(w + off[4], 0, 32, s));      // db max2 (2 floats) | flag count at +16
   IBL_CUDA_OK(cudaMemsetAsync(gate, 0xFF, (size_t)m * 4, s));      // orderable +max: no gate yet
   rows_f16_kernel<<<m, 256, 0, s>>>(q, d, qp, qa);
   rows_f16_kernel<<<n, 256, 0, s>>>(db, d, dp, da);
-  dist_colmax_kernel<<<cdiv(n_valid, 256) < 64 ? cdiv(n_valid, 256) : 64, 256, 0, s>>>(da, n_valid, dmax2);
   IBL_CUDA_OK(cudaGetLastError());
+  IBL_RET(launch_dist_colmax(&da->x, &da->z, 4, n_valid, dmax2, s));
 
   CUtensorMap ma, mb;
   {
@@ -725,7 +835,6 @@ int launch_dist_topk_1pass(const float* q, int m, const float* db, int n, int n_
     IBL_CUDA_OK(cudaFuncSetAttribute(gemm2_f16_top16_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, D1Cfg<1>::SMEM));
     IBL_CUDA_OK(cudaFuncSetAttribute(gemm2_f16_top16_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, D1Cfg<2>::SMEM));
     IBL_CUDA_OK(cudaFuncSetAttribute(dist_finish_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
-    IBL_CUDA_OK(cudaFuncSetAttribute(dist_exact_chunk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
     attr_done.mark();
   }
   const int pairs = device_sm_count() / 2;
@@ -753,24 +862,17 @@ int launch_dist_topk_1pass(const float* q, int m, const float* db, int n, int n_
   dist_finish_kernel<<<m, 128, qsm, s>>>(f);
   IBL_CUDA_OK(cudaGetLastError());
 
-  ExactArgs x{};
-  x.q = q; x.db = db; x.q_aux = qa; x.db_aux = da; x.m = m; x.d = d; x.n_valid = n_valid; x.k = k;
-  x.nchunks = cdiv(n_valid, DX_CHUNK); x.idx_base = idx_base; x.flag_count = fcount; x.flag_list = flist;
-  x.scratch = scratch; x.out_dist = out_dist; x.out_idx = out_idx;
-  dist_exact_chunk_kernel<<<device_sm_count() * 2, 256, qsm, s>>>(x);     // exits at once when nothing is listed
-  dist_exact_merge_kernel<<<32, 128, 0, s>>>(x);
-  IBL_CUDA_OK(cudaGetLastError());
+  IBL_RET(launch_dist_exact_fallback(q, &qa->x, 4, m, db, &da->x, 4, n_valid, d, k, idx_base, fcount, flist, scratch,
+                                     out_dist, out_idx, s));
   if (launches) *launches += 7;
   return IBL_OK;
 }
 
-// test hook: number of queries the guard listed in the last call on this workspace (synchronises)
-int dist1_last_flag_count(void* ws, int m, int n, int d, int* out, cudaStream_t s) {
+// device address of the guard's counter of listed queries in a workspace of dist1_workspace_bytes(m, n, d)
+int* dist1_flag_count(void* ws, int m, int n, int d) {
   size_t off[9];
   dist1_workspace_bytes(m, n, d, off);
-  IBL_CUDA_OK(cudaMemcpyAsync(out, reinterpret_cast<uint8_t*>(ws) + off[4] + 16, sizeof(int), cudaMemcpyDeviceToHost, s));
-  IBL_CUDA_OK(cudaStreamSynchronize(s));
-  return IBL_OK;
+  return reinterpret_cast<int*>(reinterpret_cast<uint8_t*>(ws) + off[4] + 16);
 }
 
 }  // namespace ibl

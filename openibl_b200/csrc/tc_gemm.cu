@@ -496,7 +496,10 @@ int pca_tc_splits(int P, int D) {
 
 // ---- exact fp32 re-scoring of a candidate list + final ordering ---------------------------------
 // one block (128 threads) per query: dist = |q|^2 + |d|^2 - 2 q.d with an fp32 dot product, then
-// (dist, idx)-ascending sort of the kc <= 128 candidates; writes the first k_out.
+// (dist, idx)-ascending sort of the kc <= 128 candidates; writes the first k_out.  Guard: a database row that was not
+// kept has a screened distance >= s_kc (the largest screened distance kept), so its exact distance is >= s_kc - B
+// (screen_guard_bound, 3 MMAs per 16-wide K step).  Unless s_kc - B > (k-th exact distance) the query is listed for
+// the exact brute force of tc_dist1.cu.
 __device__ __forceinline__ uint32_t f32_ord(float f) {
   uint32_t u = __float_as_uint(f);
   return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
@@ -506,7 +509,7 @@ __global__ void __launch_bounds__(128)
 rescore_sort_kernel(const float* __restrict__ q, const float* __restrict__ qn,
                     const float* __restrict__ db, const float* __restrict__ dbn, int d,
                     const long long* __restrict__ cand_i, int kc, int k_out, long long idx_base,
-                    float* __restrict__ out_dist, long long* __restrict__ out_idx) {
+                    float* __restrict__ out_dist, long long* __restrict__ out_idx, const RescoreGuard gd) {
   extern __shared__ __align__(16) float qs[];   // [d]
   __shared__ unsigned long long keys[128];
   const long long row = blockIdx.x;
@@ -568,11 +571,28 @@ rescore_sort_kernel(const float* __restrict__ q, const float* __restrict__ qn,
       out_idx[row * k_out + threadIdx.x] = idx_base + (long long)(uint32_t)(key & 0xffffffffu);
     }
   }
+  if (threadIdx.x == 0 && gd.n_valid > kc) {            // with <= kc rows everything was re-scored
+    const unsigned long long ek = keys[k_out - 1];
+    bool flag = ek == ~0ull;
+    float s_kc = -INFINITY;
+    for (int c = 0; c < kc; ++c) {
+      if (cand_i[row * kc + c] < 0) flag = true;         // fewer than kc candidates: cannot happen; be safe
+      s_kc = fmaxf(s_kc, gd.cand_sd[row * kc + c]);
+    }
+    if (!flag) {
+      const uint32_t u = (uint32_t)(ek >> 32);
+      const float e_k = __uint_as_float((u & 0x80000000u) ? (u & 0x7fffffffu) : ~u);
+      const float bound = screen_guard_bound(an, __ldg(gd.q_err + row), __ldg(gd.db_max2 + 1), __ldg(gd.db_max2), d,
+                                             3 * (d / 16), 1.5411377e-5f);   // |ql||dl| <= (2^-8 (1 + 2^-8))^2 |q||d|
+      flag = !(s_kc - bound > e_k);                     // also catches NaN
+    }
+    if (flag) gd.flag_list[atomicAdd(gd.flag_count, 1)] = (int)row;
+  }
 }
 
 int launch_rescore_sort(const float* q, const float* qn, int m, const float* db, const float* dbn, int d,
                         const long long* cand_i, int kc, int k_out, long long idx_base, float* out_dist,
-                        long long* out_idx, cudaStream_t s) {
+                        long long* out_idx, const RescoreGuard& guard, cudaStream_t s) {
   IBL_REQUIRE(kc >= 1 && kc <= 128 && k_out >= 1 && k_out <= 128, "rescore: 1 <= k <= 128");
   IBL_REQUIRE(d % 4 == 0, "rescore: dim must be a multiple of 4");
   static DeviceOnce attr_done;   // the attribute is per device
@@ -582,7 +602,7 @@ int launch_rescore_sort(const float* q, const float* qn, int m, const float* db,
   }
   if (m == 0) return IBL_OK;
   rescore_sort_kernel<<<m, 128, d <= 16384 ? d * sizeof(float) : 16, s>>>(q, qn, db, dbn, d, cand_i, kc, k_out, idx_base,
-                                                       out_dist, out_idx);
+                                                       out_dist, out_idx, guard);
   IBL_CUDA_OK(cudaGetLastError());
   return IBL_OK;
 }

@@ -408,7 +408,7 @@ class Engine:
         return out_dist_host, out_idx_host
 
     def dist_flagged(self) -> int:
-        """Queries re-ranked by exact brute force in the last l2dist_topk call (-1: single-pass path not taken)."""
+        """Queries re-ranked by exact brute force in the last l2dist_topk call (-1: CUDA-core path)."""
         c = c_int()
         check(self.lib.ibl_debug_dist_flagged(self.h, byref(c), _stream(self.device)), "ibl_debug_dist_flagged")
         return c.value

@@ -11,7 +11,7 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 VARIANTS = [
-    # env, -k expression
+    # env, -k expression[, test file (default test_gpu_parity.py)]
     ({"IBL_CONV_HALO": "2"}, "conv3x3 or small or odd"),                    # halo staging on every N tile
     ({"IBL_CONV_HALO": "0", "IBL_CONV_2SM": "0"}, "conv3x3 or small or odd"),   # im2col boxes, one SM per tile
     ({"IBL_CONV_2SM": "2", "IBL_CONV_HALO": "0"}, "conv3x3 or odd"),        # SM pairs on the 128-wide tiles too
@@ -21,15 +21,26 @@ VARIANTS = [
     ({"IBL_DIST_SCREEN": "3"}, "retrieval or topk"),                         # round-1 bf16x3 screening on SM pairs
     ({"IBL_DIST_SCREEN": "3", "IBL_DIST_2SM": "0"}, "retrieval_vs_reference or topk"),   # ... on one SM
     ({"IBL_DIST_SCREEN": "3", "IBL_DIST_2SM": "0", "IBL_DIST_BN": "128", "IBL_GEMM_MC": "1"}, "retrieval_vs_reference or topk"),
+    # the crafted rankings of test_gpu_rank_rounding.py on every screening variant
+    ({"IBL_DIST_BN": "512"}, "topk or dist_flagged", "test_gpu_rank_rounding.py"),
+    ({"IBL_DIST_SCREEN": "3"}, "topk or dist_flagged", "test_gpu_rank_rounding.py"),
+    ({"IBL_DIST_SCREEN": "3", "IBL_DIST_2SM": "0"}, "topk or dist_flagged", "test_gpu_rank_rounding.py"),
 ]
 
 
+def _variant_id(v):
+    ident = ",".join(f"{k}={val}" for k, val in v[0].items())
+    return ident if len(v) == 2 else ident + ":" + v[2].replace("test_gpu_", "").replace(".py", "")
+
+
 @pytest.mark.gpu
-@pytest.mark.parametrize("env,expr", VARIANTS, ids=[",".join(f"{k}={v}" for k, v in e.items()) for e, _ in VARIANTS])
-def test_variant_matches_references(env, expr):
+@pytest.mark.parametrize("variant", VARIANTS, ids=[_variant_id(v) for v in VARIANTS])
+def test_variant_matches_references(variant):
+    env, expr = variant[:2]
+    test_file = variant[2] if len(variant) > 2 else "test_gpu_parity.py"
     child_env = dict(os.environ)
     child_env.update(env)
-    r = subprocess.run([sys.executable, "-m", "pytest", os.path.join(ROOT, "tests", "test_gpu_parity.py"), "-q", "-x",
+    r = subprocess.run([sys.executable, "-m", "pytest", os.path.join(ROOT, "tests", test_file), "-q", "-x",
                         "-k", expr, "-p", "no:cacheprovider"], cwd=ROOT, env=child_env, capture_output=True, text=True,
                        timeout=600)
     tail = (r.stdout + r.stderr)[-2000:]
